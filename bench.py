@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W      # our arm, N GPUs (weak scaling)
     python bench.py --impl reference --gpus 1 --steps K --warmup W      # reference arm: CPU path on host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs bench_outputs/RUN   # + the last timed step's outputs as .npy
 
 Workload (BASELINE.json configs[1]): one step = forward of a batch of 32 synthetic 512x384 pairs through
 ViT-L encoder / 2x ViT-B decoder / DPT heads ("ViTLarge_BaseDecoder_512_dpt"), random-init weights.  With
@@ -34,6 +35,9 @@ GFLOP_PER_PAIR = 1856.8          # SURVEY §8d / BASELINE.md §2 (2*MAC, enc 104
 H, W = 384, 512
 PAIRS_PER_GPU = 32
 METRIC = 'image-pairs/sec (512x384, ViT-L/B+DPT)'
+DUMP_MAX_BYTES = 64 * 2**20      # --dump-outputs writes at most this much
+DUMP_SAMPLE_PX = 2**20           # pixel positions kept when the whole result would not fit (32 bytes each)
+DUMP_SEED = 0
 
 
 def peaks():
@@ -441,6 +445,28 @@ def run_reference_arm(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(outdir, r1, r2):
+    """--dump-outputs: the result of the last timed step, as packed.forward() hands it to its caller, written as
+    outdir/<name>.npy (float32).  When the whole result exceeds DUMP_MAX_BYTES, every array keeps the same DUMP_SAMPLE_PX pixel
+    positions, drawn with DUMP_SEED from the flat (pair, row, column) index and sorted: the sample depends only on the output
+    shape, so two builds run with the same arguments write arrays that compare element for element."""
+    arrays = dict(pred1_pts3d=r1['pts3d'], pred1_conf=r1['conf'], pred2_pts3d_in_other_view=r2['pts3d'], pred2_conf=r2['conf'])
+    n_px = int(np.prod(r1['pts3d'].shape[:3]))
+    full = sum(t.numel() * t.element_size() for t in arrays.values()) <= DUMP_MAX_BYTES - 4096     # (room for the .npy headers)
+    if not full:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n_px, min(DUMP_SAMPLE_PX, n_px), replace=False))
+        idx = torch.from_numpy(idx).to(r1['pts3d'].device)
+    os.makedirs(outdir, exist_ok=True)
+    shapes = {}
+    for name, t in arrays.items():
+        a = t if full else t.reshape(n_px, *t.shape[3:])[idx]
+        a = a.float().cpu().numpy()
+        np.save(os.path.join(outdir, name + '.npy'), a)
+        shapes[name] = list(a.shape)
+    return dict(dir=outdir, arrays=shapes, sample=None if full else
+                f'{len(idx)} of {n_px} pixel positions, numpy default_rng({DUMP_SEED}).choice without replacement, sorted')
+
+
 def ncu_traffic():
     """dram__bytes_read.sum + dram__bytes_write.sum per launch of the dominant kernels, as recorded from `ncu --set full`
     captures in profiles/ncu_traffic.json (each entry names its capture file and the commit it was taken at).  The bench
@@ -483,7 +509,13 @@ def main():
     ap.add_argument('--pairs', type=int, default=PAIRS_PER_GPU, help='pairs per GPU per step')
     ap.add_argument('--skip-cpu-baseline', action='store_true')
     ap.add_argument('--skip-cloud-opt', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write the outputs of the last one (rank 0) to '
+                    'DIR/<name>.npy, float32, at most 64 MB in all (a fixed, seeded sample of pixel positions when larger)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
     args.warmup = max(args.warmup, 0)
     if args.impl == 'reference':
         return run_reference_arm(args)
@@ -527,8 +559,10 @@ def main():
             gather.wait()
 
     W_ = max(args.warmup, 3)
+    # the last result stays referenced, in the warm-up too, so that the allocator has cached the same two output sets
+    # before the timed loop starts
     for _ in range(W_):
-        step()
+        last = step()
     drain()
     torch.cuda.synchronize()
     if world > 1:
@@ -539,11 +573,13 @@ def main():
         torch.cuda.synchronize()
         e0.record()
         for _ in range(args.steps):
-            step()
+            last = step()
         drain()
         e1.record()
         torch.cuda.synchronize()
     launches = _lib.launch_count()
+    dumped = dump_outputs(args.dump_outputs, *last) if args.dump_outputs and rank == 0 else None
+    del last
     ms = torch.tensor([e0.elapsed_time(e1)], device=device)
     if world > 1:
         dist.barrier()
@@ -617,6 +653,8 @@ def main():
                 clocks=clocks, e2e=e2e, gpu_launches=int(launches),
                 roofline=build_roofline(prof, pk, value, world),
                 kernels=kern)
+    if dumped:
+        line['dump_outputs'] = dumped
     # GPU sections first, CPU baselines last (the GPU would otherwise idle down while the host cores run the oracle)
     if world == 1 and not args.skip_cloud_opt:
         del packed, net, imgs

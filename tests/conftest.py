@@ -8,15 +8,18 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, 'tests', 'golden')
-REFERENCE = '/root/reference'
+
+from golden.make_reference_records import digest  # noqa: E402,F401  (sha256 of dtype, shape and bytes)
 
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA B200 device (run on the GPU box with -m gpu)')
 
 
-def has_reference():
-    return os.path.isdir(os.path.join(REFERENCE, 'dust3r'))
+def reference_records():
+    """What the unmodified reference returned for the comparisons of the CPU suite (tests/golden/make_reference_records.py)."""
+    import numpy as np
+    return np.load(os.path.join(GOLDEN, 'reference_records.npz'))
 
 
 @pytest.fixture(scope='session')

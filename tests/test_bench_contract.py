@@ -63,3 +63,39 @@ def test_build_roofline_on_a_recorded_breakdown():
     # a class the table has no capture for: traffic stays null
     odd = bench.build_roofline({'some_kernel': dict(count=1, ms=1.0, flops=1e12, bytes=0.0)}, pk, 1.0, 1)
     assert odd['traffic'] is None and odd['traffic_note'] is None and odd['achieved'] == 1000.0
+
+
+def test_dump_outputs_whole_or_fixed_sample_within_the_limit(tmp_path, monkeypatch):
+    """--dump-outputs: the arrays as returned when they fit; otherwise the same seeded pixel positions in every array and every
+    run, float32, within DUMP_MAX_BYTES."""
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import torch
+    import bench
+    assert bench.DUMP_SAMPLE_PX * 32 + 4 * 4096 <= bench.DUMP_MAX_BYTES
+    g = torch.Generator().manual_seed(0)
+    B, H, W = 2, 8, 12
+    r1 = dict(pts3d=torch.randn((B, H, W, 3), generator=g), conf=torch.rand((B, H, W), generator=g))
+    r2 = dict(pts3d=torch.randn((B, H, W, 3), generator=g), conf=torch.rand((B, H, W), generator=g))
+    names = dict(pred1_pts3d=r1['pts3d'], pred1_conf=r1['conf'], pred2_pts3d_in_other_view=r2['pts3d'], pred2_conf=r2['conf'])
+    info = bench.dump_outputs(str(tmp_path / 'full'), r1, r2)
+    assert info['sample'] is None and sorted(os.listdir(tmp_path / 'full')) == sorted(n + '.npy' for n in names)
+    for n, t in names.items():
+        a = np.load(tmp_path / 'full' / (n + '.npy'))
+        assert a.dtype == np.float32 and np.array_equal(a, t.numpy())
+    monkeypatch.setattr(bench, 'DUMP_MAX_BYTES', 4096 + 100 * 32)
+    monkeypatch.setattr(bench, 'DUMP_SAMPLE_PX', 50)
+    for run in ('a', 'b'):
+        info = bench.dump_outputs(str(tmp_path / run), r1, r2)
+        assert info['sample'] and sum(os.path.getsize(tmp_path / run / f) for f in os.listdir(tmp_path / run)) <= bench.DUMP_MAX_BYTES
+    idx = np.sort(np.random.default_rng(bench.DUMP_SEED).choice(B * H * W, 50, replace=False))
+    for n, t in names.items():
+        a, b = np.load(tmp_path / 'a' / (n + '.npy')), np.load(tmp_path / 'b' / (n + '.npy'))
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+        assert np.array_equal(a, t.reshape(B * H * W, *t.shape[3:]).numpy()[idx]), n
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--gpus', '1', '--steps', '0', '--warmup', '0'],
+                       capture_output=True, text=True, cwd=ROOT, timeout=120)
+    assert r.returncode == 2 and '--steps must be at least 1' in r.stderr

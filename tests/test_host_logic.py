@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, has_reference
+from conftest import GOLDEN, digest, reference_records
 from dust3r_b200.config import vitl_512_dpt, vitl_224_linear, state_dict_spec
 from dust3r_b200.image_pairs import make_pairs
 
@@ -84,76 +84,79 @@ def test_optimizer_host_objects_on_cpu():
     assert out['pred1']['pts3d'].device.type == 'cpu'
 
 
-@pytest.mark.skipif(not has_reference(), reason='reference not mounted')
 def test_optimizer_init_matches_reference_draws():
-    """Same torch seed -> same initial parameters as the reference constructor (optimizer.py:29-33)."""
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(GOLDEN), '..', 'oracle', 'roma_stub'))
-    sys.path.insert(0, '/root/reference')
+    """Same torch seed -> same initial parameters as the reference constructor (optimizer.py:29-33), whose draws are recorded
+    in tests/golden/reference_records.npz."""
     import copy
-    from dust3r.cloud_opt import global_aligner as ref_aligner, GlobalAlignerMode as RefMode
     from dust3r_b200.cloud_opt import global_aligner, GlobalAlignerMode
     from dust3r_b200.utils.synth import synth_pair_predictions
+    gold = reference_records()
     n, H, W = 3, 16, 32
     edges = [(i, j) for i in range(n) for j in range(i)]
     out = synth_pair_predictions(n, edges, H, W, seed=2)
     torch.manual_seed(123)
-    ref = ref_aligner(copy.deepcopy(out), 'cpu', mode=RefMode.PointCloudOptimizer, verbose=False)
-    torch.manual_seed(123)
     net = global_aligner(copy.deepcopy(out), 'cpu', mode=GlobalAlignerMode.PointCloudOptimizer, verbose=False)
     for k in ('pw_poses', 'im_depthmaps', 'im_poses', 'im_focals', 'im_pp'):
-        assert torch.equal(getattr(ref, k).data, getattr(net, k).data), k
-    for a, b in zip(ref.get_pts3d(), net.get_pts3d()):
-        assert torch.allclose(a, b, atol=1e-5, rtol=1e-5)
-    assert torch.allclose(ref.get_pw_poses(), net.get_pw_poses(), atol=1e-6)
+        assert torch.equal(torch.from_numpy(gold[f'init_draws|{k}']), getattr(net, k).data), k
+    pts = net.get_pts3d()
+    assert len(pts) == len([k for k in gold.files if k.startswith('init_draws|pts3d|')])
+    for i, b in enumerate(pts):
+        assert torch.allclose(torch.from_numpy(gold[f'init_draws|pts3d|{i}']), b, atol=1e-5, rtol=1e-5)
+    assert torch.allclose(torch.from_numpy(gold['init_draws|get_pw_poses']), net.get_pw_poses(), atol=1e-6)
 
 
 def test_geometry_helpers_match_live_reference():
-    """xy_grid / geotrf / inv / depthmap_to_pts3d / depthmap_to_(absolute_)camera_coordinates against the reference's
-    dust3r/utils/geometry.py on random inputs (CPU), every calling convention the two hot paths use."""
-    import pytest
-    from conftest import has_reference
-    if not has_reference():
-        pytest.skip('reference not mounted')
-    import sys
-    import numpy as np
-    import torch
-    sys.path.insert(0, '/root/reference')
-    import dust3r.utils.geometry as ref
+    """xy_grid / geotrf / inv / depthmap_to_pts3d / depthmap_to_(absolute_)camera_coordinates against what the reference's
+    dust3r/utils/geometry.py returns on the same random inputs (CPU; recorded in tests/golden/reference_records.npz), every
+    calling convention the two hot paths use."""
     import dust3r_b200.utils.geometry as mine
+    gold = reference_records()
+
+    def ref(key, a):
+        """The recorded reference output for `key`, after checking that `a` has its type, dtype and shape."""
+        b = gold[f'geometry|{key}']
+        assert type(a) is (torch.Tensor if str(gold[f'geometry|{key}|type']) == 'torch' else np.ndarray), key
+        assert a.dtype == (torch.from_numpy(b).dtype if torch.is_tensor(a) else b.dtype) and tuple(a.shape) == b.shape, key
+        return torch.from_numpy(b) if torch.is_tensor(a) else b
     g = torch.Generator().manual_seed(0)
-    for kw in (dict(), dict(origin=(2, 3)), dict(homogeneous=True), dict(unsqueeze=0), dict(cat_dim=0)):
-        a, b = mine.xy_grid(7, 5, device='cpu', **kw), ref.xy_grid(7, 5, device='cpu', **kw)
-        assert type(a) is type(b) and torch.equal(a, b), kw
+    for i, kw in enumerate((dict(), dict(origin=(2, 3)), dict(homogeneous=True), dict(unsqueeze=0), dict(cat_dim=0))):
+        a = mine.xy_grid(7, 5, device='cpu', **kw)
+        assert torch.equal(a, ref(f'xy_grid|{i}|cpu', a)), kw
         if 'unsqueeze' not in kw:      # (the reference's numpy branch cannot unsqueeze)
-            a, b = mine.xy_grid(7, 5, **kw), ref.xy_grid(7, 5, **kw)          # device=None -> numpy
-            assert type(a) is type(b) and np.array_equal(a, b), kw
+            a = mine.xy_grid(7, 5, **kw)          # device=None -> numpy
+            assert np.array_equal(a, ref(f'xy_grid|{i}|none', a)), kw
     T = torch.randn((3, 4, 4), generator=g)
     T[:, 3] = torch.tensor([0., 0, 0, 1])
     P = torch.randn((3, 6, 5, 3), generator=g)
-    assert torch.equal(mine.geotrf(T, P), ref.geotrf(T, P))
-    assert torch.equal(mine.geotrf(T[0], P[0]), ref.geotrf(T[0], P[0]))
+    a = mine.geotrf(T, P)
+    assert torch.equal(a, ref('geotrf|batched', a))
+    a = mine.geotrf(T[0], P[0])
+    assert torch.equal(a, ref('geotrf|single', a))
     K = torch.tensor([[30., 0, 16], [0, 31, 12], [0, 0, 1]])
-    assert torch.equal(mine.geotrf(K, P[0], norm=1, ncol=2), ref.geotrf(K, P[0], norm=1, ncol=2))
-    assert np.allclose(mine.geotrf(T[0].numpy(), P[0].numpy()), ref.geotrf(T[0].numpy(), P[0].numpy()))
-    assert torch.equal(mine.inv(T), ref.inv(T)) and np.array_equal(mine.inv(T[0].numpy()), ref.inv(T[0].numpy()))
+    a = mine.geotrf(K, P[0], norm=1, ncol=2)
+    assert torch.equal(a, ref('geotrf|K', a))
+    a = mine.geotrf(T[0].numpy(), P[0].numpy())
+    assert np.allclose(a, ref('geotrf|numpy', a))
+    a, b = mine.inv(T), mine.inv(T[0].numpy())
+    assert torch.equal(a, ref('inv|torch', a)) and np.array_equal(b, ref('inv|numpy', b))
     depth = torch.rand((2, 6, 5), generator=g) + 0.5
-    for focal in (torch.rand((2, 1, 6, 5), generator=g) + 20, torch.rand((2, 2, 6, 5), generator=g) + 20):
+    for f, focal in enumerate((torch.rand((2, 1, 6, 5), generator=g) + 20, torch.rand((2, 2, 6, 5), generator=g) + 20)):
         pp = torch.tensor([[2.5, 3.0], [2.0, 3.5]])
-        assert torch.equal(mine.depthmap_to_pts3d(depth, focal, pp=pp), ref.depthmap_to_pts3d(depth, focal, pp=pp))
-        assert torch.equal(mine.depthmap_to_pts3d(depth, focal), ref.depthmap_to_pts3d(depth, focal))
+        a = mine.depthmap_to_pts3d(depth, focal, pp=pp)
+        assert torch.equal(a, ref(f'depthmap_to_pts3d|{f}|pp', a))
+        a = mine.depthmap_to_pts3d(depth, focal)
+        assert torch.equal(a, ref(f'depthmap_to_pts3d|{f}|nopp', a))
     d = depth[0].numpy()
     d[0, 0] = 0
-    for fn in ('depthmap_to_camera_coordinates',):
-        xa, ma = getattr(mine, fn)(d, K.numpy())
-        xb, mb = getattr(ref, fn)(d, K.numpy())
-        assert np.array_equal(xa, xb) and np.array_equal(ma, mb)
+    xa, ma = mine.depthmap_to_camera_coordinates(d, K.numpy())
+    assert np.array_equal(xa, ref('depthmap_to_camera_coordinates|X', xa))
+    assert np.array_equal(ma, ref('depthmap_to_camera_coordinates|mask', ma))
     pose = np.eye(4, dtype=np.float32)
     pose[:3, :3] = np.float32([[0, -1, 0], [1, 0, 0], [0, 0, 1]])
     pose[:3, 3] = (1, 2, 3)
     xa, ma = mine.depthmap_to_absolute_camera_coordinates(d, K.numpy(), pose)
-    xb, mb = ref.depthmap_to_absolute_camera_coordinates(d, K.numpy(), pose)
-    assert np.allclose(xa, xb, atol=1e-6) and np.array_equal(ma, mb)
+    assert np.allclose(xa, ref('depthmap_to_absolute_camera_coordinates|X', xa), atol=1e-6)
+    assert np.array_equal(ma, ref('depthmap_to_absolute_camera_coordinates|mask', ma))
 
 
 def test_stream_work_items_cover_every_slot_once_and_balance():
@@ -196,20 +199,15 @@ def test_stream_work_items_cover_every_slot_once_and_balance():
 
 
 def test_find_reciprocal_matches_host_path_matches_live_reference():
-    """utils/geometry.py:345-361 (scipy cKDTree on the CPU, like the reference); the CUDA path is checked against this one in
-    tests/test_scene_ops_gpu.py."""
-    import numpy as np
-    from conftest import has_reference
-    if not has_reference():
-        pytest.skip('reference not mounted')
-    import sys
-    sys.path.insert(0, '/root/reference')
-    from dust3r.utils.geometry import find_reciprocal_matches as ref
+    """utils/geometry.py:345-361 (scipy cKDTree on the CPU, like the reference; its result recorded in
+    tests/golden/reference_records.npz); the CUDA path is checked against this one in tests/test_scene_ops_gpu.py."""
     from dust3r_b200.utils.geometry import find_reciprocal_matches as mine
+    gold = reference_records()
     rng = np.random.default_rng(0)
     P1 = rng.standard_normal((700, 3)).astype(np.float32)
     P2 = np.concatenate((P1[:400] + 0.01 * rng.standard_normal((400, 3)).astype(np.float32), rng.standard_normal((150, 3)).astype(np.float32)))
-    a, b = ref(P1, P2), mine(P1, P2)
+    assert digest(P1) + digest(P2) == str(gold['reciprocal|inputs']), 'inputs differ from the recorded ones'
+    a, b = [gold[f'reciprocal|{k}'] for k in range(3)], mine(P1, P2)
     assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and int(a[2]) == int(b[2]) > 300
 
 
@@ -217,10 +215,9 @@ def test_load_model_and_from_pretrained_on_a_reference_format_checkpoint(tmp_pat
     """dust3r/model.py:27-43, 76-85: a checkpoint is {'args': Namespace(model="AsymmetricCroCo3DStereo(...)"), 'model': state
     dict}; load_model rebuilds the network from the constructor string (ManyAR_PatchEmbed -> PatchEmbedDust3R,
     landscape_only forced to False) and loads the weights; from_pretrained(path) of an existing file does the same.  No real
-    checkpoint is available offline: a small synthetic one is written in that format (and read back by the live reference's
-    own load_model when it is mounted)."""
+    checkpoint is available offline: a small synthetic one is written in that format; the state dict the reference's own
+    load_model reads back from it is recorded in tests/golden/reference_records.npz (one digest per tensor)."""
     import argparse
-    from conftest import has_reference
     from dust3r_b200.config import ModelConfig
     from dust3r_b200.model import AsymmetricCroCo3DStereo, load_model
     from dust3r_b200.utils.synth import synth_state_dict
@@ -243,17 +240,9 @@ def test_load_model_and_from_pretrained_on_a_reference_format_checkpoint(tmp_pat
         assert torch.equal(got[k], src), k
     net2 = AsymmetricCroCo3DStereo.from_pretrained(path)
     assert all(torch.equal(a, b) for a, b in zip(net2.state_dict().values(), got.values()))
-    if has_reference():
-        import sys
-        sys.path.insert(0, '/root/reference')
-        from dust3r.model import load_model as ref_load_model
-        # torch >= 2.6 defaults torch.load to weights_only=True, which rejects the Namespace every DUSt3R checkpoint stores:
-        # allow it for the reference's own (unmodified) loader
-        with torch.serialization.safe_globals([argparse.Namespace]):
-            ref = ref_load_model(path, 'cpu', verbose=False)
-        rsd = ref.state_dict()
-        assert set(rsd) == set(got)
-        assert all(torch.equal(rsd[k], got[k]) for k in got)
+    gold = reference_records()
+    assert sorted(got) == gold['load_model|keys'].tolist()
+    assert [digest(got[k]) for k in sorted(got)] == gold['load_model|digests'].tolist()
 
 
 @pytest.mark.parametrize('imshapes,n_edges', [([(384, 512)] * 8, 28), ([(32, 48), (48, 32), (16, 64), (64, 64)], 5), ([(8, 8), (24, 40)], 1)])

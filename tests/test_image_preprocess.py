@@ -1,8 +1,8 @@
 """load_images preprocessing (SURVEY §8f rank 4; dust3r/utils/image.py:62-128), CPU side:
 
   * oracle/image_oracle.py (integer restatement of Pillow's resize + crop + torchvision ImgNorm) is pinned bit-exactly against
-    Pillow / torchvision themselves, the unmodified reference's load_images (when /root/reference is mounted) and the
-    committed golden fixture tests/golden/load_images.npz (reference outputs);
+    Pillow / torchvision themselves, the unmodified reference's load_images (its outputs recorded as digests in
+    tests/golden/reference_records.npz) and the committed golden fixture tests/golden/load_images.npz (reference outputs);
   * the product's host-side tables (dust3r_b200/utils/image.py) equal the oracle's;
   * the per-thread bodies of the CUDA kernels (dust3r_b200/csrc/resample_core.h) are compiled for the HOST
     (tests/native/resample_host.cpp, g++) and run over every thread index of the launches: bit-exact against the host PIL
@@ -12,13 +12,12 @@ import ctypes
 import os
 import shutil
 import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, REFERENCE, ROOT, has_reference
+from conftest import GOLDEN, ROOT, digest, reference_records
 from dust3r_b200.utils import image as img_mod
 from dust3r_b200.utils.synth import synth_photo
 from oracle import image_oracle as io
@@ -92,22 +91,20 @@ def test_oracle_equals_golden_reference_outputs():
         assert out.shape == ref.shape and np.array_equal(out, ref), k
 
 
-@pytest.mark.skipif(not has_reference(), reason='reference tree not mounted')
 def test_oracle_and_host_port_equal_live_reference_load_images(tmp_path):
-    sys.path.insert(0, REFERENCE)
-    try:
-        from dust3r.utils.image import load_images as ref_load_images
-    finally:
-        sys.path.remove(REFERENCE)
+    """The reference's load_images on the same PNG files, recorded in tests/golden/reference_records.npz (the image as a
+    digest: ours must equal it bit for bit, and the oracle must equal ours)."""
+    gold = reference_records()
     for k, (h, w, size, sq) in enumerate(CASES):
+        ref = lambda key: gold[f'load_images|{k}|{key}']
         photo = synth_photo(h, w, seed=10 + k)
+        assert digest(photo) == str(ref('photo')), ('synthetic photo differs from the recorded one', h, w)
         path = _write_png(tmp_path, photo, f'{k}.png')
-        ref = ref_load_images([path], size=size, square_ok=sq, verbose=False)[0]
         ours = img_mod.load_images([path], size=size, square_ok=sq, verbose=False)[0]
         out, true_shape = io.load_image_oracle(photo, size, sq)
-        assert torch.equal(ours['img'], ref['img']) and np.array_equal(ours['true_shape'], ref['true_shape'])
-        assert np.array_equal(out, ref['img'].numpy()) and np.array_equal(true_shape, ref['true_shape']), (h, w, size, sq)
-        assert ours['idx'] == ref['idx'] and ours['instance'] == ref['instance']
+        assert digest(ours['img']) == str(ref('img')) and np.array_equal(ours['true_shape'], ref('true_shape'))
+        assert np.array_equal(out, ours['img'].numpy()) and np.array_equal(true_shape, ref('true_shape')), (h, w, size, sq)
+        assert ours['idx'] == int(ref('idx')) and ours['instance'] == str(ref('instance'))
 
 
 # ------------------------------------------------------------------------------------------------ the GPU code, on the host
@@ -190,15 +187,10 @@ def test_load_images_folder_threads_keep_the_sequential_contract(tmp_path, capsy
             assert torch.equal(a['img'], b['img']) and np.array_equal(a['true_shape'], b['true_shape'])
             assert a['idx'] == b['idx'] and a['instance'] == b['instance']
     assert [v['idx'] for v in seq] == list(range(len(shapes))) and lines_seq.count(' - adding im') == len(shapes)
-    if has_reference():
-        sys.path.insert(0, REFERENCE)
-        try:
-            from dust3r.utils.image import load_images as ref_load_images
-        finally:
-            sys.path.remove(REFERENCE)
-        ref = ref_load_images(str(tmp_path), size=64, verbose=False)
-        assert len(ref) == len(seq)
-        for a, b in zip(seq, ref):
-            assert torch.equal(a['img'], b['img']) and np.array_equal(a['true_shape'], b['true_shape']) and a['instance'] == b['instance']
+    # the reference's load_images on the same folder (recorded in tests/golden/reference_records.npz)
+    gold = reference_records()
+    assert [digest(a['img']) for a in seq] == gold['load_images_folder|img'].tolist()
+    assert np.array_equal(np.concatenate([a['true_shape'] for a in seq]), gold['load_images_folder|true_shape'])
+    assert [a['instance'] for a in seq] == gold['load_images_folder|instance'].tolist()
     with pytest.raises(AssertionError):
         img_mod.load_images([os.path.join(str(tmp_path), 'readme.txt')], size=64, verbose=False)

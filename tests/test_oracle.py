@@ -1,19 +1,15 @@
-"""The oracles against (a) the committed golden vectors made by the reference itself and (b) the live
-reference when /root/reference is mounted.  CPU only."""
+"""The oracles against the committed golden vectors made by the reference itself.  CPU only."""
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, ROOT, has_reference
+from conftest import GOLDEN, digest, reference_records
 from dust3r_b200.utils.synth import synth_state_dict, synth_images, synth_pair_predictions
 from dust3r_b200.image_pairs import make_pairs
 from oracle.forward_oracle import forward_oracle
 from oracle.align_oracle import AlignProblem, init_params, align_oracle
-
-sys.path.insert(0, os.path.join(ROOT, 'tests', 'golden'))
 
 
 def _small_cfgs():
@@ -122,30 +118,24 @@ def test_align_oracle_matches_reference_golden(variant, dist, schedule):
     assert np.allclose(final['im_focals'].numpy(), gold[key + '|focals'], atol=2e-4)
 
 
-@pytest.mark.skipif(not has_reference(), reason='reference not mounted')
 def test_forward_oracle_bit_matches_live_reference():
-    sys.path.insert(0, '/root/reference')
+    """A symmetrised batch (the reference's half-encoder path) against the reference model's outputs, recorded at a fixed
+    quarter of the pixels in tests/golden/reference_records.npz."""
     from dust3r_b200.config import ModelConfig
-    import importlib
-    mg = importlib.import_module('make_golden')
+    gold = reference_records()
     cfg = ModelConfig(img_size=(64, 64), enc_embed_dim=128, enc_depth=2, enc_num_heads=2, dec_embed_dim=64,
                       dec_depth=10, dec_num_heads=1, head_type='dpt', landscape_only=False)
-    m = mg.ref_model(cfg)
     sd = synth_state_dict(cfg, seed=21)
-    m.load_state_dict(sd, strict=True)
     imgs = synth_images(4, 48, 64, seed=9)
     img1 = torch.cat([imgs[0]['img'], imgs[1]['img']])
     img2 = torch.cat([imgs[1]['img'], imgs[0]['img']])
-    ts = torch.tensor([[48, 64]] * 2)
-    v1 = dict(img=img1, true_shape=ts, instance=['0', '1'])
-    v2 = dict(img=img2, true_shape=ts, instance=['1', '0'])   # symmetrised batch -> half-encoder path
-    with torch.no_grad():
-        r1, r2 = m(v1, v2)
+    assert digest(img1) + digest(img2) == str(gold['forward_sym|inputs']), 'synthetic inputs differ from the recorded ones'
     o1, o2 = forward_oracle(sd, cfg, img1, img2, ['0', '1'], ['1', '0'])
-    assert torch.allclose(r1['pts3d'], o1['pts3d'], rtol=1e-5, atol=1e-6)
-    assert torch.allclose(r1['conf'], o1['conf'], rtol=1e-5, atol=1e-6)
-    assert torch.allclose(r2['pts3d_in_other_view'], o2['pts3d_in_other_view'], rtol=1e-5, atol=1e-6)
-    assert torch.allclose(r2['conf'], o2['conf'], rtol=1e-5, atol=1e-6)
+    px = torch.from_numpy(gold['forward_sym|px'])
+    for got, key in ((o1['pts3d'], 'pts3d'), (o1['conf'], 'conf1'), (o2['pts3d_in_other_view'], 'pts3d_in_other_view'),
+                     (o2['conf'], 'conf2')):
+        ref = torch.from_numpy(gold[f'forward_sym|{key}'])
+        assert torch.allclose(ref, got.reshape(2, 48 * 64, -1)[:, px], rtol=1e-5, atol=1e-6), key
 
 
 @pytest.mark.parametrize('name', ['small_linear', 'small_dpt'])
