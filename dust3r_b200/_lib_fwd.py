@@ -54,6 +54,24 @@ def declare(lib):
     lib.d3r_conv3x3_bf16.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, u32, vp]
     lib.d3r_attention_hd64.restype = C.c_int
     lib.d3r_attention_hd64.argtypes = [vp, i64, vp, i64, vp, i64, vp, i64, i32, i32, i32, i32, f32, vp]
+    lib.d3r_convT_bf16.restype = C.c_int
+    lib.d3r_convT_bf16.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp]
+    lib.d3r_conv3x3_head_tail.restype = C.c_int
+    lib.d3r_conv3x3_head_tail.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, f32, f32, vp]
+    lib.d3r_layernorm_bf16.restype = C.c_int
+    lib.d3r_layernorm_bf16.argtypes = [vp, vp, vp, vp, i32, i32, f32, vp]
+    lib.d3r_upsample2x_bf16.restype = C.c_int
+    lib.d3r_upsample2x_bf16.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp]
+    lib.d3r_im2col_3x3_s2_bf16.restype = C.c_int
+    lib.d3r_im2col_3x3_s2_bf16.argtypes = [vp, vp, i32, i32, i32, i32, vp]
+    lib.d3r_patch_im2col16.restype = C.c_int
+    lib.d3r_patch_im2col16.argtypes = [vp, vp, i32, i32, i32, vp]
+    lib.d3r_gather_images_bf16.restype = C.c_int
+    lib.d3r_gather_images_bf16.argtypes = [vp, vp, vp, i32, i32, i32, vp]
+    lib.d3r_cast_f32_bf16.restype = C.c_int
+    lib.d3r_cast_f32_bf16.argtypes = [vp, vp, i64, vp]
+    lib.d3r_linear_head_postprocess.restype = C.c_int
+    lib.d3r_linear_head_postprocess.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, i32, f32, f32, vp]
     lib.d3r_set_gemm_impl.restype = None
     lib.d3r_set_gemm_impl.argtypes = [i32]
     lib.d3r_set_attention_impl.restype = None

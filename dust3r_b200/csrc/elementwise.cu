@@ -307,3 +307,33 @@ int linear_head_postprocess(const float* feat, float* pts3d, float* conf, int B,
 
 }  // namespace ew
 }  // namespace d3r
+
+// ---- building blocks exported through the C ABI (unit tests; forward.cu calls the ew:: functions) ----
+using namespace d3r;
+
+extern "C" int d3r_layernorm_bf16(const float* x, const float* g, const float* b, void* out, int32_t M, int32_t C, float eps, void* stream) {
+  return ew::layernorm(x, g, b, out, nullptr, M, C, eps, (cudaStream_t)stream);
+}
+extern "C" int d3r_upsample2x_bf16(const void* x, void* out, int32_t B, int32_t H, int32_t W, int32_t C, int32_t Ho, int32_t Wo, void* stream) {
+  return ew::upsample2x_bf16(x, out, B, H, W, C, Ho, Wo, (cudaStream_t)stream);
+}
+extern "C" int d3r_im2col_3x3_s2_bf16(const void* x, void* out, int32_t B, int32_t H, int32_t W, int32_t C, void* stream) {
+  return ew::im2col_3x3_s2_bf16(x, out, B, H, W, C, (cudaStream_t)stream);
+}
+extern "C" int d3r_patch_im2col16(const float* img, void* out, int32_t B, int32_t H, int32_t W, void* stream) {
+  return ew::patch_im2col16(img, out, B, H, W, (cudaStream_t)stream);
+}
+extern "C" int d3r_gather_images_bf16(const void* in, void* out, const int32_t* map_dev, int32_t n_out, int32_t rows_per_img, int32_t C,
+                                      void* stream) {
+  return ew::gather_images_bf16(in, out, map_dev, n_out, rows_per_img, C, (cudaStream_t)stream);
+}
+extern "C" int d3r_cast_f32_bf16(const float* x, void* out, int64_t n, void* stream) {
+  D3R_CHECK_ARG(n >= 0, "cast: negative length");
+  return ew::cast_f32_bf16(x, out, (size_t)n, (cudaStream_t)stream);
+}
+extern "C" int d3r_linear_head_postprocess(const float* feat, float* pts3d, float* conf, int32_t B, int32_t gh, int32_t gw, int32_t nch,
+                                           int32_t depth_mode, int32_t conf_mode, float cmin, float cmax, void* stream) {
+  D3R_CHECK_ARG(feat && pts3d && (nch == 3 || nch == 4), "linear head: null buffer or nch=%d not 3 / 4", nch);
+  D3R_CHECK_ARG(nch == 3 || conf_mode == 0 || conf, "linear head: conf_mode %d without a conf buffer", conf_mode);
+  return ew::linear_head_postprocess(feat, pts3d, conf, B, gh, gw, nch, depth_mode, conf_mode, cmin, cmax, (cudaStream_t)stream);
+}

@@ -84,12 +84,7 @@ static int conv3(const Ctx& c, const void* x, const d3r_linear& w, int B, int H,
 
 // k == stride transposed convolution: rows = input pixels, columns = (ky,kx,co)
 static int convT(const Ctx& c, const void* x, const d3r_linear& w, int B, int h, int wd, int Cin, int Cout, int k, void* out) {
-  Params p{};
-  p.M = B * h * wd; p.N = k * k * Cout; p.K = Cin;
-  p.flags = gemm::F_CONVT | (w.b ? gemm::F_BIAS : 0);
-  p.out = out; p.bias = w.b; p.ldo = 0;
-  p.tk = k; p.th_in = h; p.tw_in = wd; p.tCout = Cout;
-  return gemm::gemm_bf16(x, Cin, w.w, p, c.st);
+  return gemm::convT_bf16(x, w.w, w.b, out, B, h, wd, Cin, Cout, k, c.st);
 }
 
 // ---- encoder ---------------------------------------------------------------------------------
@@ -235,16 +230,8 @@ static int run_dpt(const Ctx& c, Arena& ar, const d3r_dpt_head& hd, const void* 
   const int Hp = Hs[0] * 2, Wp = Ws[0] * 2;
   RC(conv3(c, path, hd.head0, B, Hp, Wp, F, 128, h0, 0));
   RC(ew::upsample2x_bf16(h0, h1, B, Hp, Wp, 128, Hf, Wf, c.st));
-  {
-    Params p{};
-    p.flags = gemm::F_HEAD_FINAL | (hd.head2.b ? gemm::F_BIAS : 0);
-    p.bias = hd.head2.b;
-    p.w4 = hd.head4_w; p.b4 = hd.head4_b;
-    p.pts3d = pts3d; p.conf = conf;
-    p.depth_mode = m.depth_mode; p.conf_mode = (m.nch > 3 && conf) ? m.conf_mode : 0;
-    p.conf_min = m.conf_min; p.conf_max = m.conf_max;
-    RC(gemm::conv3x3_bf16(h1, hd.head2.w, B, Hf, Wf, 128, 128, p, c.st));
-  }
+  RC(gemm::conv3x3_head_tail(h1, hd.head2.w, hd.head2.b, hd.head4_w, hd.head4_b, pts3d, m.nch > 3 ? conf : nullptr, B, Hf, Wf,
+                             m.depth_mode, m.conf_mode, m.conf_min, m.conf_max, c.st));
   return D3R_OK;
 }
 

@@ -207,6 +207,34 @@ int conv3x3_bf16(const void* x_nhwc, const void* w_packed, int B, int H, int W, 
   return dispatch(bn, ta, tb, p, total, st);
 }
 
+int convT_bf16(const void* x_nhwc, const void* w_packed, const float* bias, void* out, int B, int h, int w, int Cin, int Cout, int k,
+               cudaStream_t st) {
+  D3R_CHECK_ARG(x_nhwc && w_packed && out, "convT: null buffer");
+  D3R_CHECK_ARG(B > 0 && h > 0 && w > 0 && k > 0, "convT: bad shape");
+  // the epilogue scatters 32-column chunks: each must lie inside one (ky, kx) tap
+  D3R_CHECK_ARG(Cout % 32 == 0, "convT: Cout=%d must be a multiple of 32", Cout);
+  Params p{};
+  p.M = B * h * w; p.N = k * k * Cout; p.K = Cin;
+  p.flags = F_CONVT | (bias ? F_BIAS : 0);
+  p.out = out; p.bias = bias; p.ldo = 0;
+  p.tk = k; p.th_in = h; p.tw_in = w; p.tCout = Cout;
+  return gemm_bf16(x_nhwc, Cin, w_packed, p, st);
+}
+
+int conv3x3_head_tail(const void* x_nhwc, const void* w_packed, const float* bias, const float* w4, const float* b4, float* pts3d,
+                      float* conf, int B, int H, int W, int depth_mode, int conf_mode, float conf_min, float conf_max, cudaStream_t st) {
+  D3R_CHECK_ARG(w4 && b4 && pts3d, "head tail: null buffer");
+  D3R_CHECK_ARG(depth_mode >= 0 && depth_mode <= 2 && conf_mode >= 0 && conf_mode <= 2, "head tail: bad postprocess mode");
+  Params p{};
+  p.flags = F_HEAD_FINAL | (bias ? F_BIAS : 0);
+  p.bias = bias;
+  p.w4 = w4; p.b4 = b4;
+  p.pts3d = pts3d; p.conf = conf;
+  p.depth_mode = depth_mode; p.conf_mode = conf ? conf_mode : 0;
+  p.conf_min = conf_min; p.conf_max = conf_max;
+  return conv3x3_bf16(x_nhwc, w_packed, B, H, W, 128, 128, p, st);
+}
+
 }  // namespace gemm
 }  // namespace d3r
 
@@ -238,4 +266,16 @@ extern "C" int d3r_conv3x3_bf16(const void* x_nhwc, const void* w_packed, void* 
   p.out = out; p.out2 = out2; p.add0 = add0; p.add1 = add1; p.bias = bias;
   D3R_CHECK_ARG(!(flags & (gemm::F_CONVT | gemm::F_HEAD_FINAL | gemm::F_ROPE)), "conv3x3: unsupported flag");
   return gemm::conv3x3_bf16(x_nhwc, w_packed, B, H, W, Cin, Cout, p, (cudaStream_t)stream);
+}
+
+extern "C" int d3r_convT_bf16(const void* x_nhwc, const void* w_packed, const float* bias, void* out, int32_t B, int32_t h, int32_t w,
+                              int32_t Cin, int32_t Cout, int32_t k, void* stream) {
+  return gemm::convT_bf16(x_nhwc, w_packed, bias, out, B, h, w, Cin, Cout, k, (cudaStream_t)stream);
+}
+
+extern "C" int d3r_conv3x3_head_tail(const void* x_nhwc, const void* w_packed, const float* bias, const float* w4, const float* b4,
+                                     float* pts3d, float* conf, int32_t B, int32_t H, int32_t W, int32_t depth_mode, int32_t conf_mode,
+                                     float conf_min, float conf_max, void* stream) {
+  return gemm::conv3x3_head_tail(x_nhwc, w_packed, bias, w4, b4, pts3d, conf, B, H, W, depth_mode, conf_mode, conf_min, conf_max,
+                                 (cudaStream_t)stream);
 }

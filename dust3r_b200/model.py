@@ -293,6 +293,22 @@ class AsymmetricCroCo3DStereo(nn.Module, _HubMixin, **_hub_kwargs):
         return res1, res2
 
 
+def pack_conv3x3(w):
+    """(Cout, Cin, 3, 3) Conv2d weight -> [Cout][ky][kx][Cin]: the B operand of the implicit-GEMM 3x3 conv."""
+    return w.permute(0, 2, 3, 1).contiguous()
+
+
+def pack_conv3x3_s2(w):
+    """(Cout, Cin, 3, 3) Conv2d weight -> [Cout][(ky*3+kx)*Cin + ci]: the GEMM operand over d3r_im2col_3x3_s2_bf16 rows."""
+    return pack_conv3x3(w).reshape(w.shape[0], -1)
+
+
+def pack_convT(w):
+    """(Cin, Cout, k, k) ConvTranspose2d weight (k == stride) -> [(ky*k+kx)*Cout + co][ci]: the B operand of d3r_convT_bf16."""
+    ci, co, k, _ = w.shape
+    return w.permute(2, 3, 1, 0).reshape(k * k * co, ci).contiguous()
+
+
 class _PackedModel:
     """Device-side operand buffers + the ctypes `d3r_model` descriptor pointing at them."""
 
@@ -322,16 +338,12 @@ class _PackedModel:
         def norm(prefix):
             return CNorm(f32(sd[prefix + '.weight']), f32(sd[prefix + '.bias']))
 
-        def conv3(prefix):     # (Cout,Cin,3,3) -> [Cout][ky][kx][Cin]
-            w = sd[prefix + '.weight'].permute(0, 2, 3, 1).contiguous()
+        def conv3(prefix):
             bias = sd.get(prefix + '.bias')
-            return CLinear(bf(w), f32(bias) if bias is not None else None)
+            return CLinear(bf(pack_conv3x3(sd[prefix + '.weight'])), f32(bias) if bias is not None else None)
 
-        def convT(prefix):     # (Cin,Cout,k,k) -> [(ky*k+kx)*Cout + co][ci]
-            w = sd[prefix + '.weight']
-            ci, co, k, _ = w.shape
-            wp = w.permute(2, 3, 1, 0).reshape(k * k * co, ci).contiguous()
-            return CLinear(bf(wp), f32(sd[prefix + '.bias']))
+        def convT(prefix):
+            return CLinear(bf(pack_convT(sd[prefix + '.weight'])), f32(sd[prefix + '.bias']))
 
         m = CModel()
         m.enc_dim, m.enc_depth, m.enc_heads = E, cfg.enc_depth, cfg.enc_num_heads
@@ -400,8 +412,8 @@ class _PackedModel:
                     hd.layer_rn[k] = conv3(f'{p}.scratch.layer{k + 1}_rn')
                 hd.act0_up = convT(f'{p}.act_postprocess.0.1')
                 hd.act1_up = convT(f'{p}.act_postprocess.1.1')
-                w = sd[f'{p}.act_postprocess.3.1.weight'].permute(0, 2, 3, 1).reshape(768, -1)  # [Cout][tap*Cin]
-                hd.act3_down = lin(None, w=w, b=sd[f'{p}.act_postprocess.3.1.bias'])
+                hd.act3_down = lin(None, w=pack_conv3x3_s2(sd[f'{p}.act_postprocess.3.1.weight']),
+                                   b=sd[f'{p}.act_postprocess.3.1.bias'])
                 for r in range(4):
                     q = f'{p}.scratch.refinenet{r + 1}'
                     f = hd.refine[r]

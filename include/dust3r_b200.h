@@ -239,10 +239,61 @@ int d3r_conv3x3_bf16(const void* x_nhwc_dev, const void* w_packed_dev, void* out
                      int32_t Cin, int32_t Cout, uint32_t flags, void* stream);
 
 /* softmax(q k^T * scale) v, head dim 64, bf16 in/out, fp32 softmax (croco/models/blocks.py:94-112,
- * 146-169).  q rows at (b*Nq+i)*ldq + h*64, k/v rows at (b*Nk+j)*ld{k,v} + h*64, out like q. */
+ * 146-169).  q rows at (b*Nq+i)*ldq + h*64, k/v rows at (b*Nk+j)*ld{k,v} + h*64, out like q.
+ * Range: the exponent reference of a row moves lazily (DESIGN.md section 4); a key whose scaled logit leads the keys before
+ * it by 86 or more (natural-log units) overflows fp32 and the row's output is NaN (measured on a B200; finite up to 84). */
 int d3r_attention_hd64(const void* q_dev, int64_t ldq, const void* k_dev, int64_t ldk, const void* v_dev, int64_t ldv,
                        void* out_dev, int64_t ldo, int32_t B, int32_t heads, int32_t Nq, int32_t Nk, float scale,
                        void* stream);
+
+/* ConvTranspose2d with kernel == stride == k (act_postprocess 0 / 1, dpt_head.py via croco/models/dpt_block.py) as a
+ * GEMM whose epilogue scatters every (ky,kx,co) column to its output pixel.  x: (B,h,w,Cin) bf16 NHWC;
+ * w_packed: [(ky*k+kx)*Cout + co][Cin] bf16; bias [Cout] fp32 or NULL; out: (B,h*k,w*k,Cout) bf16 NHWC.
+ * Cin % 8 == 0, Cout % 32 == 0 (a 32-column chunk of the epilogue must stay inside one (ky,kx) tap). */
+int d3r_convT_bf16(const void* x_nhwc_dev, const void* w_packed_dev, const float* bias_dev, void* out_dev, int32_t B, int32_t h,
+                   int32_t w, int32_t Cin, int32_t Cout, int32_t k, void* stream);
+
+/* Last DPT conv with the head tail fused into its epilogue: 3x3 conv 128 -> 128 (+ bias) -> ReLU -> 1x1 conv to 4
+ * channels (w4 fp32 [4][128], b4 fp32 [4]; always four rows, row 3 is the confidence logit) -> postprocess
+ * (heads/postprocess.py: depth_mode 0 linear, 1 square, 2 exp; conf_mode 0 none, 1 exp, 2 sigmoid, range
+ * [conf_min, conf_max]).  x: (B,H,W,128) bf16 NHWC; w_packed: [128][9][128] bf16; pts3d: (B,H,W,3) fp32;
+ * conf: (B,H,W) fp32, or NULL for no confidence output (conf_mode is then ignored). */
+int d3r_conv3x3_head_tail(const void* x_nhwc_dev, const void* w_packed_dev, const float* bias_dev, const float* w4_dev,
+                          const float* b4_dev, float* pts3d_dev, float* conf_dev, int32_t B, int32_t H, int32_t W,
+                          int32_t depth_mode, int32_t conf_mode, float conf_min, float conf_max, void* stream);
+
+/* LayerNorm over the last dimension, fp32 in, bf16 out: out[m] = (x[m] - mean) / sqrt(var + eps) * g + b (biased
+ * variance, like nn.LayerNorm).  x: [M][C] fp32, g, b: [C] fp32.  C % 4 == 0, C <= 2048. */
+int d3r_layernorm_bf16(const float* x_dev, const float* g_dev, const float* b_dev, void* out_dev, int32_t M, int32_t C, float eps,
+                       void* stream);
+
+/* Bilinear x2 upsampling with align_corners=True of x (B,H,W,C) bf16 NHWC onto the (2H, 2W) grid, of which the first
+ * Ho x Wo pixels are written to out (B,Ho,Wo,C) (Ho <= 2H, Wo <= 2W: the crop of refinenet4, dpt_head.py:57).
+ * C % 8 == 0 and C / 8 a power of two. */
+int d3r_upsample2x_bf16(const void* x_dev, void* out_dev, int32_t B, int32_t H, int32_t W, int32_t C, int32_t Ho, int32_t Wo,
+                        void* stream);
+
+/* im2col of a 3x3 stride-2 pad-1 convolution: x (B,H,W,C) bf16 NHWC -> out [B*Ho*Wo][9][C] bf16 (tap = ky*3+kx, zeros
+ * outside the image), Ho = (H-1)/2+1, Wo = (W-1)/2+1.  C % 8 == 0. */
+int d3r_im2col_3x3_s2_bf16(const void* x_dev, void* out_dev, int32_t B, int32_t H, int32_t W, int32_t C, void* stream);
+
+/* Patch-embedding im2col, 16 x 16 patches: img (B,3,H,W) fp32 -> out [B*(H/16)*(W/16)][3*16*16] bf16 with column
+ * c*256 + py*16 + px (the flattening of the Conv2d weight).  H % 16 == 0, W % 16 == 0. */
+int d3r_patch_im2col16(const float* img_dev, void* out_dev, int32_t B, int32_t H, int32_t W, void* stream);
+
+/* Row gather by image: out[i*rows_per_img + r] = in[map[i]*rows_per_img + r] for i < n_out, rows of C bf16.
+ * map_dev: int32 [n_out] (device).  C % 8 == 0. */
+int d3r_gather_images_bf16(const void* in_dev, void* out_dev, const int32_t* map_dev, int32_t n_out, int32_t rows_per_img,
+                           int32_t C, void* stream);
+
+/* fp32 -> bf16, round to nearest even, n elements, n % 4 == 0. */
+int d3r_cast_f32_bf16(const float* x_dev, void* out_dev, int64_t n, void* stream);
+
+/* Linear head tail (heads/linear_head.py + postprocess.py): feat [B*gh*gw][nch*256] fp32 (channel-major, then
+ * py*16 + px) -> pixel shuffle -> pts3d (B,gh*16,gw*16,3) and, when nch == 4, conf (B,gh*16,gw*16) fp32.  Modes as for
+ * d3r_conv3x3_head_tail. */
+int d3r_linear_head_postprocess(const float* feat_dev, float* pts3d_dev, float* conf_dev, int32_t B, int32_t gh, int32_t gw,
+                                int32_t nch, int32_t depth_mode, int32_t conf_mode, float conf_min, float conf_max, void* stream);
 
 /* Selects the GEMM / conv kernel family: 0 = 1-CTA tcgen05 kernels, 1 = CTA-pair (cta_group::2) kernels,
  * 2 (default) = CTA-pair kernels from 4 k-blocks of 64 on (K >= 256), 1-CTA for shorter reductions. */
@@ -330,8 +381,8 @@ typedef struct d3r_dpt_head {       /* DPTOutputAdapter_fix, dust3r/heads/dpt_he
   d3r_fusion refine[4];             /* refinenet1..4                                               */
   d3r_linear head0;                 /* 3x3 256->128 packed                                         */
   d3r_linear head2;                 /* 3x3 128->128 packed                                         */
-  const float* head4_w;             /* fp32 [nch][128]                                             */
-  const float* head4_b;             /* fp32 [nch]                                                  */
+  const float* head4_w;             /* fp32 [4][128], always 4 rows: row 3 zero when nch == 3      */
+  const float* head4_b;             /* fp32 [4], entry 3 zero when nch == 3                        */
 } d3r_dpt_head;
 
 typedef struct d3r_model {

@@ -102,6 +102,32 @@ def forward_goldens():
         print('wrote', name)
 
 
+ODD_GRID_SIZES = [(48, 80), (80, 48)]   # small_dpt at 3x5 and 5x3 tokens: odd grid width and height in the DPT head
+
+
+def forward_odd_grid_goldens():
+    """small_dpt on token grids with an odd width or height, same flow as forward_goldens: the stride-2 conv of
+    act_postprocess 3 rounds the grid up and refinenet4's x2 output is cropped back to the grid (heads/dpt_head.py:57)."""
+    from dust3r.inference import inference
+    from dust3r.image_pairs import make_pairs
+    cfg = SMALL['small_dpt'][0]
+    for H, W in ODD_GRID_SIZES:
+        torch.manual_seed(0)
+        m = ref_model(cfg)
+        sd = synth_state_dict(cfg, seed=11)
+        m.load_state_dict(sd, strict=True)
+        imgs = synth_images(3, H, W, seed=5)
+        pairs = make_pairs(imgs, scene_graph='complete', prefilter=None, symmetrize=True)
+        out = inference(pairs, m, 'cpu', batch_size=4, verbose=False)
+        np.savez_compressed(os.path.join(HERE, f'forward_small_dpt_{H}x{W}.npz'),
+                            pts3d=out['pred1']['pts3d'].numpy(), conf1=out['pred1']['conf'].numpy(),
+                            pts3d_in_other_view=out['pred2']['pts3d_in_other_view'].numpy(),
+                            conf2=out['pred2']['conf'].numpy(),
+                            idx1=np.int64(out['view1']['idx']), idx2=np.int64(out['view2']['idx']),
+                            img_sum=np.float64([float(i['img'].double().sum()) for i in imgs]))
+        print('wrote odd grid', (H, W), out['pred1']['pts3d'].shape)
+
+
 def forward_mixed_goldens():
     from dust3r.inference import inference
     from dust3r.image_pairs import make_pairs
@@ -232,3 +258,5 @@ if __name__ == '__main__':
             forward_goldens()
         if 'forward' in what or 'mixed' in what:
             forward_mixed_goldens()
+        if 'forward' in what or 'odd' in what:
+            forward_odd_grid_goldens()

@@ -39,6 +39,59 @@ def _rel(a, b):
     return float((a - b).norm() / b.norm().clamp_min(1e-12))
 
 
+def _attention(q, ldq, k, ldk, v, ldv, B, Hh, Nq, Nk, scale=0.125):
+    """runs d3r_attention_hd64 on row-strided q / k / v views (row r of q at q.data_ptr() + r * ldq elements)"""
+    from dust3r_b200 import _lib
+    lib = _lib.get_lib()
+    out = torch.full((B, Nq, Hh, 64), float('nan'), dtype=torch.bfloat16, device=q.device)
+    _lib.check(lib.d3r_attention_hd64(q.data_ptr(), ldq, k.data_ptr(), ldk, v.data_ptr(), ldv, out.data_ptr(), Hh * 64,
+                                      B, Hh, Nq, Nk, scale, _lib.stream_ptr()))
+    torch.cuda.synchronize()
+    return out
+
+
+def _attention_ratio(out, q, k, v, scale=0.125):
+    """worst |o - o_ref| / (2^-8 sum_j p_j |v_j| + 2^-8 |o_ref|) with the exact (float64) softmax p: one bf16 rounding of
+    every p_j and one of the output.  q, k, v: (B, N, heads, 64) bf16 views."""
+    qf, kf, vf = [t.double().permute(0, 2, 1, 3) for t in (q, k, v)]
+    p = torch.softmax(qf @ kf.transpose(-1, -2) * scale, dim=-1)
+    ref = p @ vf
+    bound = 2 ** -8 * (p @ vf.abs()) + 2 ** -8 * ref.abs()
+    err = (out.double().permute(0, 2, 1, 3) - ref).abs()
+    return float((err / bound).max())
+
+
+def _attention_cases(dev, g):
+    """(label, q, ldq, k, ldk, v, ldv, B, heads, Nq, Nk): contiguous q / k / v, also with spread logits; the forward's
+    layouts -- self-attention
+    slices of one [B N][3C] qkv buffer, cross-attention q [B Nq][C] with k / v slices of one [B Nk][2C] buffer; key counts
+    around the 16-key first-block reference and the 64 / 128-key blocks, 1 to 129 queries, 12 and 16 heads"""
+    def rnd(*shape):
+        return torch.randn(shape, generator=g).to(dev).bfloat16()
+    for (B, Hh, Nq, Nk) in [(2, 3, 24, 24), (1, 2, 196, 196), (2, 4, 768, 768), (1, 2, 100, 37), (3, 1, 65, 130),
+                            (6, 16, 768, 768), (40, 8, 100, 137)]:
+        q, k, v = rnd(B, Nq, Hh, 64), rnd(B, Nk, Hh, 64), rnd(B, Nk, Hh, 64)
+        yield 'contiguous', q, Hh * 64, k, Hh * 64, v, Hh * 64, B, Hh, Nq, Nk
+    # spread logits (q x 4: scaled logits of standard deviation 4): a few keys carry p, so an error in the exponential of
+    # one key or in the scale moves the output by a share of |v_i - v_j| instead of averaging out over many keys.  Nk = 2-4
+    # are ragged blocks, 128 / 256 whole ones (where tc3 takes every 4th key pair's exponential on the FMA pipe).
+    for Nk in (2, 3, 4, 128, 256):
+        q, k, v = 4 * rnd(2, 128, 4, 64).float(), rnd(2, Nk, 4, 64), rnd(2, Nk, 4, 64)
+        yield 'spread', q.bfloat16(), 256, k, 256, v, 256, 2, 4, 128, Nk
+    for (B, Hh, N) in [(2, 12, 196), (2, 16, 768), (3, 12, 129)]:
+        Cc = Hh * 64
+        qkv = rnd(B * N, 3 * Cc)
+        yield 'qkv', qkv[:, :Cc], 3 * Cc, qkv[:, Cc:2 * Cc], 3 * Cc, qkv[:, 2 * Cc:], 3 * Cc, B, Hh, N, N
+    n = 0
+    for Nq in (1, 127, 128, 129):
+        for Nk in (1, 15, 16, 17, 63, 64, 65, 127, 128, 129, 257):
+            Hh = 12 if n % 2 == 0 else 16
+            n += 1
+            Cc = Hh * 64
+            q, kv = rnd(2 * Nq, Cc), rnd(2 * Nk, 2 * Cc)
+            yield 'q+kv', q, Cc, kv[:, :Cc], 2 * Cc, kv[:, Cc:], 2 * Cc, 2, Hh, Nq, Nk
+
+
 @pytest.mark.timeout(600)
 @pytest.mark.parametrize('impl', [2, 3])
 def test_attention_matches_torch(cuda_device, impl):
@@ -46,24 +99,20 @@ def test_attention_matches_torch(cuda_device, impl):
     lib = _lib.get_lib()
     lib.d3r_set_attention_impl(impl)
     g = torch.Generator().manual_seed(0)
-    # the last two shapes give the persistent kernel (impl 2) several tiles per CTA, one of them with ragged key blocks
-    for (B, Hh, Nq, Nk) in [(2, 3, 24, 24), (1, 2, 196, 196), (2, 4, 768, 768), (1, 2, 100, 37), (3, 1, 65, 130),
-                            (6, 16, 768, 768), (40, 8, 100, 137)]:
-        q = torch.randn((B, Nq, Hh, 64), generator=g).to(cuda_device).bfloat16()
-        k = torch.randn((B, Nk, Hh, 64), generator=g).to(cuda_device).bfloat16()
-        v = torch.randn((B, Nk, Hh, 64), generator=g).to(cuda_device).bfloat16()
-        out = torch.full((B, Nq, Hh, 64), float('nan'), dtype=torch.bfloat16, device=cuda_device)
-        ld = Hh * 64
-        _lib.check(lib.d3r_attention_hd64(q.data_ptr(), ld, k.data_ptr(), ld, v.data_ptr(), ld, out.data_ptr(), ld,
-                                          B, Hh, Nq, Nk, 0.125, _lib.stream_ptr()))
-        torch.cuda.synchronize()
-        qf, kf, vf = [t.float().permute(0, 2, 1, 3) for t in (q, k, v)]
-        ref = (torch.softmax(qf @ kf.transpose(-1, -2) * 0.125, dim=-1) @ vf).permute(0, 2, 1, 3)
-        assert torch.isfinite(out.float()).all()
-        err = (out.float() - ref).abs().max().item()
-        lib.d3r_set_attention_impl(3) if err >= 2e-2 else None
-        assert err < 2e-2, (impl, B, Hh, Nq, Nk, err)
-    lib.d3r_set_attention_impl(3)
+    worst = 0.0
+    try:
+        # the contiguous (6, 16, 768) and (40, 8, 100, 137) shapes give the persistent kernel (impl 2) several tiles per CTA,
+        # one of them with ragged key blocks
+        for label, q, ldq, k, ldk, v, ldv, B, Hh, Nq, Nk in _attention_cases(cuda_device, g):
+            out = _attention(q, ldq, k, ldk, v, ldv, B, Hh, Nq, Nk)
+            assert torch.isfinite(out.float()).all(), (impl, label, B, Hh, Nq, Nk)
+            view = lambda t, n: t.reshape(B, n, Hh, 64)
+            r = _attention_ratio(out, view(q, Nq), view(k, Nk), view(v, Nk))
+            worst = max(worst, r)
+            assert r <= 1.0, (impl, label, B, Hh, Nq, Nk, r)
+    finally:
+        lib.d3r_set_attention_impl(3)
+    print(f'attention impl {impl}: worst error / bound {worst:.3e}')
 
 
 @pytest.mark.timeout(600)
@@ -75,6 +124,7 @@ def test_attention_growing_scores_move_the_reference(cuda_device, impl):
     lib = _lib.get_lib()
     lib.d3r_set_attention_impl(impl)
     g = torch.Generator().manual_seed(1)
+    worst = 0.0
     try:
         for (B, Hh, Nq, Nk) in [(2, 2, 256, 768), (1, 3, 130, 700)]:
             q = torch.randn((B, Nq, Hh, 64), generator=g)
@@ -84,30 +134,73 @@ def test_attention_growing_scores_move_the_reference(cuda_device, impl):
             k = k * ramp + 0.35 * ramp * q.mean(dim=1, keepdim=True)
             v = torch.randn((B, Nk, Hh, 64), generator=g)
             q, k, v = [t.to(cuda_device).bfloat16() for t in (q, k, v)]
-            out = torch.full((B, Nq, Hh, 64), float('nan'), dtype=torch.bfloat16, device=cuda_device)
-            ld = Hh * 64
-            _lib.check(lib.d3r_attention_hd64(q.data_ptr(), ld, k.data_ptr(), ld, v.data_ptr(), ld, out.data_ptr(), ld,
-                                              B, Hh, Nq, Nk, 0.125, _lib.stream_ptr()))
-            torch.cuda.synchronize()
-            qf, kf, vf = [t.float().permute(0, 2, 1, 3) for t in (q, k, v)]
+            qf, kf = [t.float().permute(0, 2, 1, 3) for t in (q, k)]
             logits = qf @ kf.transpose(-1, -2) * 0.125
             # the scenario is only meaningful if row maxima really outgrow the first block's by more than the headroom
             growth = (logits.max(dim=-1).values - logits[..., :128].max(dim=-1).values) * 1.4427
             assert float(growth.max()) > 16
-            ref = (torch.softmax(logits, dim=-1) @ vf).permute(0, 2, 1, 3)
+            out = _attention(q, Hh * 64, k, Hh * 64, v, Hh * 64, B, Hh, Nq, Nk)
             assert torch.isfinite(out.float()).all()
-            err = (out.float() - ref).abs().max().item()
-            assert err < 3e-2, (impl, B, Hh, Nq, Nk, err)
+            r = _attention_ratio(out, q, k, v)
+            worst = max(worst, r)
+            assert r <= 1.0, (impl, B, Hh, Nq, Nk, r)
+    finally:
+        lib.d3r_set_attention_impl(3)
+    print(f'attention impl {impl}, growing scores: worst error / bound {worst:.3e}')
+
+
+def _dominant_key_inputs(dev, delta, where, Nq=130, Nk=700, Hh=2, seed=3):
+    """q[0] = 8 in every row, the rest small noise: key `where` (k[0] = delta) leads every other key by delta in scaled-logit
+    units (scale 0.125); where = 'jump': every key from 300 on leads the keys before it by delta."""
+    g = torch.Generator().manual_seed(seed)
+    q = 0.1 * torch.randn((1, Nq, Hh, 64), generator=g)
+    q[..., 0] = 8.0
+    k = 0.1 * torch.randn((1, Nk, Hh, 64), generator=g)
+    if where == 'jump':
+        k[:, 300:, :, 0] += float(delta)
+    else:
+        k[:, where] = 0
+        k[:, where, :, 0] = float(delta)
+    v = torch.randn((1, Nk, Hh, 64), generator=g)
+    return [t.to(dev).bfloat16() for t in (q, k, v)]
+
+
+DOMINANT_KEY_PLACES = [5, 40, 100, 200, 690, 'jump']   # key 690 lies in the last (ragged) 128-key block of 700
+
+
+@pytest.mark.timeout(600)
+@pytest.mark.parametrize('impl', [2, 3])
+@pytest.mark.parametrize('delta', [20, 60, pytest.param(100, marks=pytest.mark.xfail(
+    strict=True, reason='known limit: p of a key leading the lazy exponent reference by 86 or more overflows fp32 '
+                        '(DESIGN.md section 4)'))])
+def test_attention_dominant_key_range(cuda_device, impl, delta):
+    """One key (or, for 'jump', the whole rest of the sequence) leads by delta in scaled-logit units q.k * scale.  The kernel
+    takes its first exponent reference from the first 16 keys of each 64-key half and moves it one block late, so until it
+    moves a leading key's p = 2^(1.4427 delta).  Measured on a B200: finite and within the bound up to delta = 84; the output
+    turns to NaN from delta = 86 (the 'jump', 400 leading keys), 88 (one key in blocks 0-2; tc2 from block 1 on) and 90
+    (the last, ragged block)."""
+    from dust3r_b200 import _lib
+    lib = _lib.get_lib()
+    lib.d3r_set_attention_impl(impl)
+    try:
+        for where in DOMINANT_KEY_PLACES:
+            q, k, v = _dominant_key_inputs(cuda_device, delta, where)
+            out = _attention(q, 128, k, 128, v, 128, 1, 2, q.shape[1], k.shape[1])
+            assert torch.isfinite(out.float()).all(), (impl, delta, where)
+            r = _attention_ratio(out, q, k, v)
+            assert r <= 1.0, (impl, delta, where, r)
     finally:
         lib.d3r_set_attention_impl(3)
 
 
 @pytest.mark.timeout(900)
-@pytest.mark.parametrize('name', ['small_linear', 'small_dpt'])
+@pytest.mark.parametrize('name', ['small_linear', 'small_dpt', 'small_dpt_48x80', 'small_dpt_80x48'])
 def test_forward_matches_oracle_and_reference_golden(cuda_device, name):
+    """small_dpt_48x80 / _80x48: odd token grid width / height, where the stride-2 conv of act_postprocess 3 rounds up and
+    refinenet4's x2 output is cropped back to the grid"""
     from dust3r_b200.inference import inference
-    from oracle.forward_oracle import forward_oracle
-    cfg, H, W = _small_cfgs()[name]
+    from test_oracle import _forward_case
+    cfg, H, W = _forward_case(name)
     net, sd = _build(cfg, 11, cuda_device)
     imgs = synth_images(3, H, W, seed=5)
     pairs = make_pairs(imgs, scene_graph='complete', prefilter=None, symmetrize=True)

@@ -25,6 +25,15 @@ def _small_cfgs():
     return ns['SMALL']
 
 
+def _forward_case(name):
+    """(cfg, H, W) of a forward golden: a SMALL entry, or 'small_dpt_{H}x{W}' for the odd token grids of make_golden.py"""
+    if name in _small_cfgs():
+        return _small_cfgs()[name]
+    base, size = name.rsplit('_', 1)
+    H, W = (int(v) for v in size.split('x'))
+    return _small_cfgs()[base][0], H, W
+
+
 def _run_oracle_like_inference(cfg, sd, pairs, batch_size):
     """inference() semantics (inference.py:55-72): batches of `batch_size` pairs, outputs concatenated."""
     res = {k: [] for k in ('pts3d', 'conf1', 'pts3d_in_other_view', 'conf2')}
@@ -38,9 +47,10 @@ def _run_oracle_like_inference(cfg, sd, pairs, batch_size):
     return {k: torch.cat(v) for k, v in res.items()}
 
 
-@pytest.mark.parametrize('name', ['small_dpt', 'small_linear'])
+@pytest.mark.parametrize('name', ['small_dpt', 'small_linear', 'small_dpt_48x80', 'small_dpt_80x48'])
 def test_forward_oracle_matches_reference_golden(name):
-    cfg, H, W = _small_cfgs()[name]
+    """small_dpt_48x80 / _80x48: token grids of odd width / height (3 x 5, 5 x 3) through the DPT head"""
+    cfg, H, W = _forward_case(name)
     gold = np.load(os.path.join(GOLDEN, f'forward_{name}.npz'))
     sd = synth_state_dict(cfg, seed=11)
     imgs = synth_images(3, H, W, seed=5)
